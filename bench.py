@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W              (N = 1: plain python; N > 1: torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py ... --dump-outputs DIR                     (also writes what the last timed step computed)
 
 Workload (BASELINE.json `metric`: "Mpix/s encode+decode 8K RGB q75"):  one STEP = encode one 7680x4320
 RGB 4:4:4 frame at q75, restart interval 36, non-interleaved, then decode the JPEG just produced.
@@ -36,6 +37,20 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 W, H, QUALITY, RST = 7680, 4320, 75, 36
 WORKLOADS = {"8k": (7680, 4320, 36), "4k": (3840, 2160, 24), "hd": (1920, 1080, 24), "16k": (15360, 8640, 36)}
+DUMP_VALUES = 1 << 22   # values kept per dumped array: three arrays of at most 16 MiB each in float32
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: each array as DIR/<name>.npy in float32 (exact for the u8 / i16 outputs of the codec).  An array of more
+    than DUMP_VALUES values is reduced to the values at DUMP_VALUES positions drawn by a fixed seed, so that two builds run
+    with the same arguments can be compared output for output."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a).reshape(-1)
+        if a.size > DUMP_VALUES:
+            a = a[np.sort(np.random.default_rng(0).integers(0, a.size, DUMP_VALUES))]
+        np.save(os.path.join(directory, name + ".npy"), a.astype(np.float32))
 
 
 def hbm_peak():
@@ -428,7 +443,12 @@ def main():
     # BASELINE.json config 5: a fixed batch of frames sharded round-robin over the ranks (strong scaling); with --batch the
     # step is the whole batch.  `--size 16k --batch 32` is the configuration the reference's north star names.
     ap.add_argument("--batch", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step of each timed path "
+                    "computed (rank 0's frame): the encoder's quantised coefficients and the decoded pixels of the resident "
+                    "path, the JPEG stream of the end-to-end path; float32 .npy files, large ones as a fixed seeded sample")
     args = ap.parse_args()
+    if args.dump_outputs and (args.batch or args.impl != "b200"):
+        ap.error("--dump-outputs applies to the single-frame workload of --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -509,6 +529,10 @@ def main():
         step_resident()
     ms_total = timed(step_resident, args.steps)
     ms_step = ms_total / args.steps
+    outputs = {}
+    if args.dump_outputs and rank == 0:   # before the per-stage timings below run the kernels again
+        outputs["coefficients"] = enc.coefficients(width, height, (lh, lv), args.interleaved)
+        outputs["pixels"] = d_out.cpu().numpy()
     value = world * npix / (ms_step * 1e-3) / 1e6
 
     # ---- per-stage times for the roofline (same stream, CUDA events, inputs > L2) ----
@@ -527,19 +551,23 @@ def main():
         p = g.api.default_parameters(QUALITY, rst, args.interleaved, args.subsampling)
         addr, size = enc.encode_raw(host_img, p, g.api.image_parameters(width, height), device=False)
         dec.decode_raw(addr, size, g.api.GPUJPEG_DECODER_OUTPUT_CUSTOM_BUFFER, h_out.data_ptr())
-        return size
+        return addr, size
 
     for _ in range(args.warmup):
-        jpeg_size = step_e2e()
+        jpeg_addr, jpeg_size = step_e2e()
     barrier()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        jpeg_size = step_e2e()
+        jpeg_addr, jpeg_size = step_e2e()
     barrier()
     dt = torch.tensor([time.perf_counter() - t0], device=dev)
     if world > 1:
         dist.all_reduce(dt, op=dist.ReduceOp.MAX)
     e2e_sync_ms = float(dt.item()) / args.steps * 1e3
+    if args.dump_outputs and rank == 0:   # the encoder's JPEG buffer stays valid until its next call
+        import ctypes
+        outputs["jpeg"] = np.ctypeslib.as_array((ctypes.c_uint8 * jpeg_size).from_address(jpeg_addr)).copy()
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---- the same calls from several host threads, one coder pair + one CUDA stream each: step n+1's H2D overlaps
     #      step n's kernels and step n-1's D2H (PCIe is full duplex).  Every step still copies its 99.5 MB in and its

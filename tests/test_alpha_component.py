@@ -1,15 +1,15 @@
 """4-component JPEGs (SURVEY section 8f rank 4: "4-component alpha"): an RGBA image encoded with comp_count = 4 keeps its
 alpha samples as a fourth component.  CPU tests: the oracle restatement against the reference's own header writer + CPU
-Huffman coder compiled in place, and the product's host writer / reader against the oracle."""
+Huffman coder compiled in place (their answers recorded in tests/golden/ref_alpha_component.json), and the product's host
+writer / reader against the oracle."""
 import ctypes as C
 
 import numpy as np
 import pytest
 
 import _oracle as o
+from _refstore import digest, want
 from _shims import hs
-
-needs_ref = pytest.mark.skipif(o.ref is None, reason="oracle/_ref not built")
 
 
 def rgba(w, h, seed=3):
@@ -24,10 +24,9 @@ CASES = [(100, 60, 85, 5, 0, (1, 1)), (100, 60, 85, 5, 1, (1, 1)), (64, 48, 75, 
          (100, 60, 80, 3, 1, (2, 2)), (101, 61, 80, 4, 0, (2, 1)), (96, 64, 70, 6, 1, (1, 2))]
 
 
-@needs_ref
 @pytest.mark.parametrize("w,h,q,rst,il,sampling", CASES)
 @pytest.mark.parametrize("internal", [o.CS_JPEG, o.CS_RGB])
-def test_four_component_stream_bytes(w, h, q, rst, il, sampling, internal):
+def test_four_component_stream_bytes(request, w, h, q, rst, il, sampling, internal):
     """SPIFF header (profile, colour space code 3 / 10), four SOF0 components with ids 1..4 / 'R','G','B','A', the fourth coded
     with the luminance tables and the first component's sampling, four scans or one interleaved scan: oracle bytes against
     the reference's header writer + CPU Huffman encoder on the same coefficients"""
@@ -38,16 +37,22 @@ def test_four_component_stream_bytes(w, h, q, rst, il, sampling, internal):
     assert jpeg[2:4].tobytes() == b"\xff\xe8" and jpeg[6:12].tobytes() == b"SPIFF\x00"
     assert o.probe(jpeg).comp_count == 4
     coef = o.coefficients(jpeg)
-    out = np.empty(4096 + coef.size * 8, np.uint8)
-    if internal == o.CS_RGB:
-        n = ref_encode_rgb4(coef, w, h, q, rst, il, out)
-    else:
-        n = o.ref.ref_encode_from_coef_ss(coef, w, h, 4, q, rst, il, sampling[0], sampling[1], out, out.size)
-    assert n > 0 and np.array_equal(out[:n], jpeg), "oracle bytes != reference header writer + CPU Huffman encoder"
-    if internal != o.CS_RGB:   # and back: the reference's CPU Huffman decoder recovers the coefficients of all four components
+
+    def live():
+        out = np.empty(4096 + coef.size * 8, np.uint8)
+        if internal == o.CS_RGB:
+            n = ref_encode_rgb4(coef, w, h, q, rst, il, out)
+        else:
+            n = o.ref.ref_encode_from_coef_ss(coef, w, h, 4, q, rst, il, sampling[0], sampling[1], out, out.size)
+        assert n > 0
+        if internal == o.CS_RGB:
+            return [digest(out[:n]), None]
         from _refcpu import ref_decode_coef
-        ref_coef = ref_decode_coef(jpeg, w, h, rst, il, comps=4, sampling=sampling)
-        assert np.array_equal(ref_coef.reshape(-1), coef), "reference CPU Huffman decoder != oracle coefficients"
+        return [digest(out[:n]), digest(ref_decode_coef(jpeg, w, h, rst, il, comps=4, sampling=sampling).reshape(-1))]
+    ref_jpeg, ref_coef = want("alpha_component", request.node.name, live)
+    assert digest(jpeg) == ref_jpeg, "oracle bytes != reference header writer + CPU Huffman encoder"
+    if internal != o.CS_RGB:   # and back: the reference's CPU Huffman decoder recovers the coefficients of all four components
+        assert digest(coef) == ref_coef, "reference CPU Huffman decoder != oracle coefficients"
     back = o.decode_any(jpeg, o.FMT_4444_P0123, o.CS_RGB).reshape(h, w, 4).astype(int)
     assert np.abs(back[:, :, :3] - img[:, :, :3]).mean() < 14 and np.abs(back[:, :, 3] - img[:, :, 3]).mean() < 8
     # without alpha on the way out: the colour samples are the same

@@ -1,20 +1,24 @@
 """GPU tests of the last pieces of SURVEY section 8f rank 4: 4-component (alpha) JPEGs, the Exif header and orientation
 metadata through the encoder / decoder options, image-file helpers through the public API -- product against the CPU
-oracle and, where oracle/_ref/libgpujpeg_refgpu.so was built, against the reference GPU library itself."""
+oracle and against the reference GPU library itself (its outputs for these inputs recorded in
+tests/golden/ref_gpu_api_surface.json, tests/_refstore.py)."""
 import ctypes as C
-import os
 
 import numpy as np
 import pytest
 
 import _oracle as o
+from _refstore import digest, want as _want
 from test_alpha_component import rgba
-from test_ref_gpu import SO, run_ref
+from test_ref_gpu import ref_file, run_ref
 
 pytestmark = pytest.mark.gpu
-have_ref = pytest.mark.skipif(not os.path.exists(SO), reason="oracle/_ref/libgpujpeg_refgpu.so not built")
 RGB, YCC = 1, 3
 FMT_RGB, FMT_RGBA = 1, 6
+
+
+def recorded(request, live):
+    return _want("gpu_api_surface", request.node.name, live)
 
 
 @pytest.mark.parametrize("w,h,q,rst,il,ss", [(640, 360, 80, 6, 0, "4:4:4"), (640, 360, 80, 6, 1, "4:4:4"), (333, 77, 90, 3, 1, "4:2:0"),
@@ -44,32 +48,33 @@ def test_four_component_jpeg_against_oracle(w, h, q, rst, il, ss):
     d.close()
 
 
-@have_ref
 @pytest.mark.parametrize("il,packed,ss", [(0, 0x11111111, (1, 1)), (1, 0x11111111, (1, 1)), (1, 0x22111122, (2, 2))])
-def test_four_component_jpeg_against_reference_gpu(tmp_path, il, packed, ss):
+def test_four_component_jpeg_against_reference_gpu(request, tmp_path, il, packed, ss):
     """the reference GPU library with comp_count = 4: its bytes == oracle == product; its decoder (RGBA out) == float
     flavour of oracle and product"""
     import gpujpeg_b200 as g
     w, h, q, rst = 640, 360, 85, 6
     img = rgba(w, h)
     src, path, dst = tmp_path / "in.raw", tmp_path / "ref.jpg", tmp_path / "out.raw"
-    img.tofile(src)
-    run_ref("encode_raw", src, FMT_RGBA, RGB, w, h, q, rst, il, path, "sub:%#x" % packed)
-    ref = np.fromfile(path, np.uint8)
+
+    def live():
+        img.tofile(src)
+        run_ref("encode_raw", src, FMT_RGBA, RGB, w, h, q, rst, il, path, "sub:%#x" % packed)
+        reply = run_ref("decode_fmt", path, RGB, g.api.GPUJPEG_PIXFMT_AUTODETECT, dst)
+        return [ref_file(path), reply["pixel_format"], ref_file(dst)]
+    ref, pixel_format, pix = recorded(request, live)
     want = o.encode_any(img, w, h, o.FMT_4444_P0123, o.CS_RGB, q, rst, il, ss, threads=4, alpha=True)
-    assert ref.size == want.size and np.array_equal(ref, want), "oracle restatement != reference GPU library output"
+    assert digest(want) == ref, "oracle restatement != reference GPU library output"
     e = g.Encoder()
     name = {(1, 1): "4:4:4", (2, 2): "4:2:0"}[ss]
     got = e.encode_samples(img.reshape(-1), w, h, FMT_RGBA, q, rst, il, color_space=RGB, subsampling=name, alpha=True)
-    assert np.array_equal(got, ref), "product != reference GPU library output"
+    assert digest(got) == ref, "product != reference GPU library output"
     e.close()
-    reply = run_ref("decode_fmt", path, RGB, g.api.GPUJPEG_PIXFMT_AUTODETECT, dst)
-    assert reply["pixel_format"] == FMT_RGBA
-    pix = np.fromfile(dst, np.uint8)
-    assert np.array_equal(pix, o.decode_any(ref, o.FMT_4444_P0123, o.CS_RGB, o.IDCT_FLOAT_GPUREF, threads=4)), "oracle != reference GPU decoder"
+    assert pixel_format == FMT_RGBA
+    assert digest(o.decode_any(want, o.FMT_4444_P0123, o.CS_RGB, o.IDCT_FLOAT_GPUREF, threads=4)) == pix, "oracle != reference GPU decoder"
     d = g.Decoder(idct="float_gpuref")
-    out, _ = d.decode_samples(ref)
-    assert np.array_equal(out, pix), "product decode != reference GPU decoder"
+    out, _ = d.decode_samples(want)
+    assert digest(out) == pix, "product decode != reference GPU decoder"
     d.close()
 
 
@@ -126,39 +131,41 @@ def test_exif_and_orientation_through_the_coders():
     e.close()
 
 
-@have_ref
 @pytest.mark.parametrize("opts", [["enc_hdr=Exif", "enc_exif_tag=DateTime=2024:02:29 12:34:56"],
                                   ["enc_exif_tag=DateTime=2024:02:29 12:34:56", "enc_metadata=orientation=90-", "enc_exif_tag=0x9286:UNDEFINED=hello"],
                                   ["enc_metadata=orientation=180"], ["enc_metadata=orientation=270-", "enc_hdr=SPIFF"]])
-def test_exif_and_orientation_against_reference_gpu(tmp_path, opts):
+def test_exif_and_orientation_against_reference_gpu(request, tmp_path, opts):
     """whole files of the reference GPU library with the same options: identical bytes (a user DateTime fixes the clock);
     the reference decoder reads the product's orientation back"""
     import gpujpeg_b200 as g
     w, h = 320, 200
     img = o.gen_image("photo", w, h)
     src, path, dst = tmp_path / "in.raw", tmp_path / "ref.jpg", tmp_path / "out.raw"
-    img.tofile(src)
-    run_ref("encode_raw", src, FMT_RGB, RGB, w, h, 80, 6, 0, path, *["opt:" + x for x in opts])
-    ref = np.fromfile(path, np.uint8)
     e = g.Encoder()
     for x in opts:
         k, _, v = x.partition("=")
         e.set_option(k, v)
     got = e.encode(img, 80, 6)
     e.close()
-    assert got.size == ref.size and np.array_equal(got, ref), "product file != reference GPU library file"
-    got.tofile(path)
-    reply = run_ref("decode_fmt", path, RGB, FMT_RGB, dst)
-    assert reply["orientation"] == list(_info(got)[1])
+
+    def live():
+        img.tofile(src)
+        run_ref("encode_raw", src, FMT_RGB, RGB, w, h, 80, 6, 0, path, *["opt:" + x for x in opts])
+        ref = ref_file(path)
+        got.tofile(path)
+        return [ref, run_ref("decode_fmt", path, RGB, FMT_RGB, dst)["orientation"]]
+    ref, orientation = recorded(request, live)
+    assert digest(got) == ref, "product file != reference GPU library file"
+    assert orientation == list(_info(got)[1])
 
 
 FILES = [("a.ppm", FMT_RGB, RGB), ("a.pgm", 0, YCC), ("a.pam", FMT_RGBA, RGB), ("a.pnm", FMT_RGB, RGB), ("a.y4m", 5, YCC), ("a.y4m", 2, 2)]
 
 
 @pytest.mark.parametrize("name,fmt,cs", FILES)
-def test_image_files_through_the_public_api(tmp_path, name, fmt, cs):
-    """gpujpeg_image_save_to_file / _get_properties / _load_from_file (pinned memory) of the product; with the reference GPU
-    library present: its files are byte-identical, it loads the product's files and answers get_properties the same"""
+def test_image_files_through_the_public_api(request, tmp_path, name, fmt, cs):
+    """gpujpeg_image_save_to_file / _get_properties / _load_from_file (pinned memory) of the product; against the reference GPU
+    library: its files are byte-identical, it loads the product's files and answers get_properties the same"""
     import gpujpeg_b200.api as api
     lib = api.lib
     w, h = 70, 50
@@ -179,16 +186,20 @@ def test_image_files_through_the_public_api(tmp_path, name, fmt, cs):
     assert np.array_equal(np.ctypeslib.as_array((C.c_uint8 * size.value).from_address(ptr.value)), raw)
     lib.gpujpeg_image_destroy.argtypes = [C.c_void_p]
     lib.gpujpeg_image_destroy(ptr)
-    if not os.path.exists(SO):
-        return
     src, ref_path, dump = tmp_path / "in.raw", tmp_path / ("ref_" + name), tmp_path / "dump.raw"
-    raw.tofile(src)
-    rc, _ = run_ref("file_save", src, ref_path, fmt, cs, w, h)
-    assert rc == 0 and open(ref_path, "rb").read() == open(path, "rb").read(), "file of the reference library differs"
-    assert run_ref("file_props", path.decode(), 1) == [0, got.width, got.height, got.color_space, got.pixel_format]
-    assert run_ref("file_load", path.decode(), dump) == [0, raw.size] and np.array_equal(np.fromfile(dump, np.uint8), raw)
-    for probe in ("x.pnm", "x.pam", "x.pgm", "x.y4m", "x.rgb", "x.i420"):   # names of files still to be written
-        want = run_ref("file_props", probe, 0)
+    probes = ("x.pnm", "x.pam", "x.pgm", "x.y4m", "x.rgb", "x.i420")   # names of files still to be written
+
+    def live():
+        raw.tofile(src)
+        rc, _ = run_ref("file_save", src, ref_path, fmt, cs, w, h)
+        return {"save": [rc, ref_file(ref_path)], "props": run_ref("file_props", path.decode(), 1),
+                "load": run_ref("file_load", path.decode(), dump) + [ref_file(dump)],
+                "probes": [run_ref("file_props", probe, 0) for probe in probes]}
+    ref = recorded(request, live)
+    assert ref["save"] == [0, digest(np.fromfile(path.decode(), np.uint8))], "file of the reference library differs"
+    assert ref["props"] == [0, got.width, got.height, got.color_space, got.pixel_format]
+    assert ref["load"] == [0, raw.size, digest(raw)]
+    for probe, want in zip(probes, ref["probes"]):
         mine = api.ImageParameters(0, 0, 0, -1, 0)
         rc = lib.gpujpeg_image_get_properties(probe.encode(), C.byref(mine), 0)
         assert [rc, mine.color_space, mine.pixel_format] == [want[0], want[3], want[4]], probe

@@ -1,7 +1,7 @@
 """Image file helpers of the public API (SURVEY section 8f rank 4: "image file I/O helpers"): PGM / PPM / PNM / PAM and Y4M.
 CPU tests: the product's gj_common.c + gj_imageio.c run over host stand-ins for CUDA (tests/_shims.py io_shim) and are held
-against the reference's own pam.c / y4m.c compiled in place (oracle/_ref/libgpujpeg_refcpu.so) and against the rules of
-its delegates (src/utils/image_delegate.c:149-340)."""
+against the reference's own pam.c / y4m.c compiled in place (oracle/_ref/libgpujpeg_refcpu.so; its answers recorded in
+tests/golden/ref_image_io.json) and against the rules of its delegates (src/utils/image_delegate.c:149-340)."""
 import ctypes as C
 import os
 
@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 
 import _oracle as o
+from _refstore import digest, want
 from _shims import io
 
 U8, P012, P0P1P2_444, P1020, P0P1P2_422, P0P1P2_420, P0123 = range(7)
@@ -49,7 +50,8 @@ def _libc_malloc(n):
     return _libc.malloc(n)
 
 
-if o.ref is not None:
+def _ref():
+    """the reference's pam.c / y4m.c (only called while recording their answers)"""
     o.ref.pam_read.argtypes = [C.c_char_p, C.POINTER(PamMeta), C.POINTER(C.c_void_p), _ALLOC]
     o.ref.pam_read.restype = C.c_bool
     o.ref.pam_write.argtypes = [C.c_char_p, C.c_uint, C.c_uint, C.c_uint, C.c_int, C.c_int, C.c_void_p, C.c_bool]
@@ -58,6 +60,11 @@ if o.ref is not None:
     o.ref.y4m_read.restype = C.c_size_t
     o.ref.y4m_write.argtypes = [C.c_char_p, C.POINTER(Y4mMeta), C.c_void_p]
     o.ref.y4m_write.restype = C.c_bool
+    return o.ref
+
+
+def _recorded(request, live):
+    return want("image_io", request.node.name, live)
 
 
 def _size(w, h, fmt):
@@ -102,7 +109,7 @@ def _rand(n, seed=1):
     ("pam", P012, RGB, 3, b"P7\nWIDTH 37\nHEIGHT 21\nDEPTH 3\nMAXVAL 255\nTUPLTYPE RGB\nENDHDR\n"),
     ("pam", P0123, RGB, 4, b"P7\nWIDTH 37\nHEIGHT 21\nDEPTH 4\nMAXVAL 255\nTUPLTYPE RGB_ALPHA\nENDHDR\n"),
 ])
-def test_netpbm_save_load(tmp_path, ext, fmt, cs, depth, head):
+def test_netpbm_save_load(request, tmp_path, ext, fmt, cs, depth, head):
     w, h = 37, 21
     data = _rand(w * h * depth)
     path = tmp_path / ("img." + ext)
@@ -115,19 +122,21 @@ def test_netpbm_save_load(tmp_path, ext, fmt, cs, depth, head):
     rc, p = _props(path)
     assert rc == 0 and (p.width, p.height, p.pixel_format) == (w, h, fmt)
     assert p.color_space == (BT601_256 if depth == 1 else RGB)
-    if o.ref is not None:
-        ref_path = tmp_path / ("ref." + ext)
-        assert o.ref.pam_write(str(ref_path).encode(), w, w, h, depth, 255, data.ctypes.data, ext != "pam")
-        assert ref_path.read_bytes() == raw                  # byte-identical files
+
+    def live():
+        ref, ref_path = _ref(), tmp_path / ("ref." + ext)
+        assert ref.pam_write(str(ref_path).encode(), w, w, h, depth, 255, data.ctypes.data, ext != "pam")
         m, ptr = PamMeta(), C.c_void_p()
-        assert o.ref.pam_read(str(path).encode(), C.byref(m), C.byref(ptr), _malloc)
-        assert (m.width, m.height, m.ch_count, m.maxval) == (w, h, depth, 255)
+        assert ref.pam_read(str(path).encode(), C.byref(m), C.byref(ptr), _malloc)
         got = np.ctypeslib.as_array(C.cast(ptr, C.POINTER(C.c_uint8)), (data.size,)).copy()
         _libc.free(ptr)
-        assert np.array_equal(got, data)
+        return [digest(np.frombuffer(ref_path.read_bytes(), np.uint8)), [m.width, m.height, m.ch_count, m.maxval], digest(got)]
+    ref_file, meta, got = _recorded(request, live)
+    assert digest(np.frombuffer(raw, np.uint8)) == ref_file              # byte-identical files
+    assert meta == [w, h, depth, 255] and got == digest(data)           # the reference reads the product's file
 
 
-def test_netpbm_headers_with_comments(tmp_path):
+def test_netpbm_headers_with_comments(request, tmp_path):
     data = _rand(5 * 4 * 3)
     p = tmp_path / "c.ppm"
     p.write_bytes(b"P6\n# made by hand\n5 # width\n 4\n#\n255\n" + data.tobytes())
@@ -141,11 +150,14 @@ def test_netpbm_headers_with_comments(tmp_path):
     assert rc == 0 and (pr.width, pr.height, pr.pixel_format) == (5, 4, P0123)
     rc, back = _load(q)
     assert rc == 0 and back.size == 80
-    if o.ref is not None:
-        for f, n in ((p, 3), (q, 4)):
+
+    def live():
+        metas = []
+        for f in (p, q):
             m = PamMeta()
-            assert o.ref.pam_read(str(f).encode(), C.byref(m), None, _ALLOC(0))
-            assert (m.width, m.height, m.ch_count, m.maxval) == (5, 4, n, 255)
+            metas.append([bool(_ref().pam_read(str(f).encode(), C.byref(m), None, _ALLOC(0))), m.width, m.height, m.ch_count, m.maxval])
+        return metas
+    assert _recorded(request, live) == [[True, 5, 4, 3, 255], [True, 5, 4, 4, 255]]
 
 
 @pytest.mark.parametrize("content,why", [
@@ -160,7 +172,7 @@ def test_netpbm_headers_with_comments(tmp_path):
     (b"P7\nWIDTH 2147483647\nHEIGHT 2147483647\nDEPTH 2147483647\nMAXVAL 255\nENDHDR\n" + bytes(64), "sizes whose product wraps"),
     (b"P6\n70000 2\n255\n" + bytes(64), "wider than a JPEG can be"),
 ])
-def test_netpbm_refused(tmp_path, content, why):
+def test_netpbm_refused(request, tmp_path, content, why):
     p = tmp_path / "bad.pnm"
     p.write_bytes(content)
     rc, _ = _load(p)
@@ -168,9 +180,9 @@ def test_netpbm_refused(tmp_path, content, why):
     if why != "samples missing":
         rc, _ = _props(p)
         assert rc < 0, why
-    if o.ref is not None and why not in ("16-bit samples", "bitmap", "sizes whose product wraps", "wider than a JPEG can be"):   # (pam.c reads those; the delegates then refuse everything but 255 levels)
+    if why not in ("16-bit samples", "bitmap", "sizes whose product wraps", "wider than a JPEG can be"):   # (pam.c reads those; the delegates then refuse everything but 255 levels)
         m, ptr = PamMeta(), C.c_void_p()
-        assert not o.ref.pam_read(str(p).encode(), C.byref(m), C.byref(ptr), _malloc), why
+        assert not _recorded(request, lambda: bool(_ref().pam_read(str(p).encode(), C.byref(m), C.byref(ptr), _malloc))), why
 
 
 def test_netpbm_save_rules(tmp_path):
@@ -188,7 +200,7 @@ def test_netpbm_save_rules(tmp_path):
     (P0P1P2_444, BT709, "444", "LIMITED", 444), (P0P1P2_420, BT601, "420", "LIMITED", 420),
 ])
 @pytest.mark.parametrize("w,h", [(32, 16), (37, 21)])
-def test_y4m_save_load(tmp_path, fmt, cs, chroma, rng, ss, w, h):
+def test_y4m_save_load(request, tmp_path, fmt, cs, chroma, rng, ss, w, h):
     n = _size(w, h, fmt)
     data = _rand(n)
     path = tmp_path / "f.y4m"
@@ -201,18 +213,21 @@ def test_y4m_save_load(tmp_path, fmt, cs, chroma, rng, ss, w, h):
     rc, p = _props(path)
     assert rc == 0 and (p.width, p.height, p.pixel_format) == (w, h, fmt)
     assert p.color_space == (BT601 if rng == "LIMITED" else BT601_256)
-    if o.ref is not None:
-        ref_path = tmp_path / "ref.y4m"
+
+    def live():
+        ref, ref_path = _ref(), tmp_path / "ref.y4m"
         m = Y4mMeta(w, h, 8, ss, rng == "LIMITED")
-        assert o.ref.y4m_write(str(ref_path).encode(), C.byref(m), data.ctypes.data)
-        assert ref_path.read_bytes() == raw
+        assert ref.y4m_write(str(ref_path).encode(), C.byref(m), data.ctypes.data)
         m2, ptr = Y4mMeta(), C.c_void_p()
-        assert o.ref.y4m_read(str(path).encode(), C.byref(m2), C.byref(ptr), _malloc) == n
-        assert (m2.width, m2.height, m2.bitdepth, m2.subsampling, m2.limited) == (w, h, 8, ss, rng == "LIMITED")
+        size = ref.y4m_read(str(path).encode(), C.byref(m2), C.byref(ptr), _malloc)
         _libc.free(ptr)
+        return [digest(np.frombuffer(ref_path.read_bytes(), np.uint8)), size, [m2.width, m2.height, m2.bitdepth, m2.subsampling, m2.limited]]
+    ref_file, size, meta = _recorded(request, live)
+    assert digest(np.frombuffer(raw, np.uint8)) == ref_file
+    assert size == n and meta == [w, h, 8, ss, rng == "LIMITED"]
 
 
-def test_y4m_foreign_headers(tmp_path):
+def test_y4m_foreign_headers(request, tmp_path):
     w, h = 6, 4
     n420 = w * h + 2 * 3 * 2
     p = tmp_path / "ff.y4m"
@@ -221,6 +236,7 @@ def test_y4m_foreign_headers(tmp_path):
     assert rc == 0 and (pr.width, pr.height, pr.pixel_format, pr.color_space) == (w, h, P0P1P2_420, BT601_256)
     rc, back = _load(p)
     assert rc == 0 and back.size == n420
+    ref_reads = {}
     for head, why in ((b"YUV4MPEG2 W6 H4 C420p10\nFRAME\n", "10 bits"), (b"YUV4MPEG2 W6 H4 C444alpha\nFRAME\n", "alpha"),
                       (b"YUV4MPEG2 W6 H4\nFRAME\n", "no chroma tag: the reference does not assume 4:2:0"),
                       (b"YUV4MPEG2 W6 H4 C420\nFRAME \n", "FRAME with parameters"), (b"YUV4MPEG W6 H4 C420\nFRAME\n", "magic"),
@@ -228,9 +244,17 @@ def test_y4m_foreign_headers(tmp_path):
         q = tmp_path / "bad.y4m"
         q.write_bytes(head + bytes(200))
         assert _props(q)[0] < 0, why
-        if o.ref is not None and why in ("no chroma tag: the reference does not assume 4:2:0", "FRAME with parameters", "magic"):
-            m = Y4mMeta()
-            assert o.ref.y4m_read(str(q).encode(), C.byref(m), None, _ALLOC(0)) == 0, why
+        if why in ("no chroma tag: the reference does not assume 4:2:0", "FRAME with parameters", "magic"):
+            ref_reads[why] = q.read_bytes()
+
+    def live():
+        m, sizes = Y4mMeta(), {}
+        for why, content in ref_reads.items():
+            q.write_bytes(content)
+            sizes[why] = _ref().y4m_read(str(q).encode(), C.byref(m), None, _ALLOC(0))
+        return sizes
+    sizes = _recorded(request, live)
+    assert sorted(sizes) == sorted(ref_reads) and not any(sizes.values()), sizes
     assert _save(tmp_path / "x.y4m", _rand(w * h * 3), w, h, P012, BT601_256)[0] != 0     # packed format
     assert _save(tmp_path / "y.y4m", _rand(w * h * 3), w, h, P0P1P2_444, RGB)[0] != 0     # RGB
 
